@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]                 # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] # the reference's CPU path
     torchrun --nproc-per-node N ... bench.py --gpus N ...               # one rank per GPU
+    python bench.py ... --dump-outputs DIR                              # + DIR/logits.npy of the last timed step
 
 One "step" = one decode token for the whole batch through all 32 layers of a random-init
 Llama-3.1-8B (library GEMMs for the projections/MLP; the 30 sparse layers run this repo's three
@@ -71,7 +72,15 @@ def parse_args():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--profile-step", action="store_true",
                     help="bracket ONE extra decode step with cudaProfilerStart/Stop (for `ncu --profile-from-start off`)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits of the last timed decode step to DIR/logits.npy (float32, (B, vocab)), so that two builds "
+                         "can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the decode step's logits: --impl ours only")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -611,7 +620,8 @@ def measure_step(args, runner, dev, rank, world, local_rank, replicas, sample_cl
         used = runner.capture(warm=3)
         launches_per_step = (ctx.launch_count - launches_before) // used
     step_fn = runner.step if args.no_graph else runner.replay
-    ids_host = torch.randint(0, vocab, (args.steps + args.warmup + 8, args.B, 1), dtype=torch.long).pin_memory()
+    ids_host = torch.randint(0, vocab, (args.steps + args.warmup + 8, args.B, 1), generator=torch.Generator().manual_seed(0),
+                             dtype=torch.long).pin_memory()
     logits_host = torch.empty((args.B, vocab), dtype=torch.float32).pin_memory()
     runner.ids.copy_(ids_host[0])
     for _ in range(args.warmup):
@@ -627,6 +637,7 @@ def measure_step(args, runner, dev, rank, world, local_rank, replicas, sample_cl
         sampler.start()
     ms_total = timed(step_fn, args.steps)
     clocks = sampler.stop() if (rank == 0 and sample_clocks) else None
+    logits = runner.logits.cpu() if args.dump_outputs else None   # what the last timed step returned (the e2e steps below advance it)
     tokens = args.B * args.steps * replicas
     value = tokens / (ms_total / 1e3)
     it = {"i": 0}
@@ -642,7 +653,19 @@ def measure_step(args, runner, dev, rank, world, local_rank, replicas, sample_cl
         e2e_step()
     ms_e2e = timed(e2e_step, args.steps)
     return dict(value=value, ms_per_step=ms_total / args.steps, e2e_value=tokens / (ms_e2e / 1e3), e2e_ms_per_step=ms_e2e / args.steps,
-                clocks=clocks, launches_per_step=launches_per_step, h2d=args.B * 8, d2h=args.B * vocab * 4)
+                clocks=clocks, launches_per_step=launches_per_step, h2d=args.B * 8, d2h=args.B * vocab * 4, logits=logits)
+
+
+def dump_outputs(out_dir: str, logits):
+    """`--dump-outputs`: the last timed step's logits as <out_dir>/logits.npy (float32).  Above 64 MB (B > 130) only a fixed,
+    seeded sample of the batch rows is kept, in ascending row order."""
+    import numpy as np
+    a = logits.float().numpy()
+    keep = (64 << 20) // a[0].nbytes
+    if a.shape[0] > keep:
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), a)
 
 
 def release_runner(runner):
@@ -758,6 +781,8 @@ def main():
     hot, roofline, _ = measure_hot_path(args, runner, dev, default_workload)
     replicas = world if (world > 1 and not tp) else 1
     r = measure_step(args, runner, dev, rank, world, local_rank, replicas)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["logits"])
 
     line = None
     if rank == 0:

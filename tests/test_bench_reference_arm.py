@@ -1,15 +1,24 @@
 """`bench.py --impl reference` (the reference's CPU operators timed on host cores) needs no GPU, so its contract is
 checked here: one JSON line with the shared keys, `impl: reference`, a `cpu_baseline` describing the run and an `e2e`
-equal to the line's own value with no host<->device bytes; under torchrun only rank 0 works and prints."""
+equal to the line's own value with no host<->device bytes; under torchrun only rank 0 works and prints.  Where the
+reference's operators were not built (oracle/_ref), the arm times the C restatement instead (`kind: port`)."""
 import json
 import os
+import socket
 import subprocess
 import sys
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_OK = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "lsh.so")) or os.path.isdir("/root/reference")
+
+
+def _free_port():
+    s = socket.socket()
+    s.bind(("127.0.0.1", 0))
+    p = s.getsockname()[1]
+    s.close()
+    return p
 
 
 def _json_lines(text: str):
@@ -40,7 +49,6 @@ def _check(line):
     assert abs(best - cb["ms_per_layer"]) < 1e-9
 
 
-@pytest.mark.skipif(not REF_OK, reason="needs oracle/_ref (built from /root/reference by __graft_entry__.build())")
 @pytest.mark.timeout(600)
 def test_reference_arm_single():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1"],
@@ -52,12 +60,11 @@ def test_reference_arm_single():
     assert lines[0]["n_gpus"] == 1 and lines[0]["steps"] == 1 and lines[0]["warmup"] == 1
 
 
-@pytest.mark.skipif(not REF_OK, reason="needs oracle/_ref (built from /root/reference by __graft_entry__.build())")
 @pytest.mark.timeout(600)
 def test_reference_arm_under_torchrun_rank0_only():
     env = dict(os.environ, MASTER_ADDR="127.0.0.1")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
-                        "--master-port", "29541", os.path.join(ROOT, "bench.py"), "--gpus", "2", "--impl", "reference", "--steps", "1",
+                        "--master-port", str(_free_port()), os.path.join(ROOT, "bench.py"), "--gpus", "2", "--impl", "reference", "--steps", "1",
                         "--warmup", "1", "--P", "6000", "--M", "8192"],   # a small context: this test is about who runs and prints
                        capture_output=True, text=True, cwd=ROOT, timeout=580, env=env)
     assert r.returncode == 0, r.stderr[-2000:]

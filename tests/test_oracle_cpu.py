@@ -1,9 +1,7 @@
 """CPU suite (`-m "not gpu"`): pins the oracle and checks the host-side plumbing.
 
   * oracle/mpig_oracle.c (the C restatement) against the committed golden vectors produced by the
-    reference's own compiled operators (tests/golden/make_golden.py), and against those operators
-    live when oracle/_ref is present (it is in the build container; on the GPU box it travels as a
-    prebuilt binary);
+    reference's own compiled operators (tests/golden/make_golden.py);
   * the selection rule and the attention math against the reference tests' torch formulas
     (library/lsh/test.py:43, library/sparse_attention/test_sparse.py:68-84);
   * the C-ABI shared library loads and exports every symbol include/magicpig_b200.h declares.
@@ -16,8 +14,8 @@ import pytest
 import torch
 
 import oracle
-from oracle import ref_loader
 from magicpig_b200 import synth, _native
+from tests.golden.make_golden import ATTN_DIMS, PROBE_CASES, attention_case_inputs, checksum, probe_case_inputs, probe_case_key
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -198,26 +196,26 @@ def test_window_and_merge_restatement():
     assert torch.allclose(om, ou, atol=1e-5) and abs(float(lm[0] - lu[0])) < 1e-4
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="oracle/_ref not built / CPU lacks AVX-512")
-@pytest.mark.parametrize("K,L,seq,delta,group,bsz", [(4, 50, 1024, 128, 4, 1), (8, 100, 1024, 128, 8, 2), (8, 50, 4096, 1024, 4, 1)])
+def load_operator_case(key: str, *inputs):
+    """The compiled reference's outputs for one case of operator_cases.npz, after checking that the seeded inputs are the
+    ones they were computed from."""
+    z = np.load(os.path.join(GOLD, "operator_cases.npz"))
+    assert checksum(*inputs) == str(z[f"{key}_input_sha256"]), "inputs differ from the ones the stored reference outputs belong to"
+    return {k[len(key) + 1:]: z[k] for k in z.files if k.startswith(key + "_")}
+
+
+@pytest.mark.parametrize("K,L,seq,delta,group,bsz", PROBE_CASES)
 def test_port_probe_vs_live_reference(K, L, seq, delta, group, bsz):
-    """library/lsh/test.py's own case shape, checked three ways: reference binary, port, torch formula."""
-    lsh_m, _, _ = ref_loader.load()
-    g = torch.Generator().manual_seed(K * 1000 + L)
+    """library/lsh/test.py's own case shape, checked three ways: the reference binary's recorded outputs
+    (tests/golden/operator_cases.npz), port, torch formula."""
     Hq = 32
     Hkv = Hq // group
-    NB, M = 1 << K, seq + delta
-    codes = torch.randint(0, NB, (bsz, Hkv, L, seq), generator=g, dtype=torch.int16)
+    M = seq + delta
+    codes, query = probe_case_inputs(K, L, seq, delta, group, bsz)
+    ref = load_operator_case(probe_case_key(K, L, seq, delta, group, bsz), codes, query)
+    results, nnz, mask = (torch.from_numpy(ref[k]) for k in ("results", "nnz", "mask"))
+    assert results.shape == mask.shape == (bsz * Hq, M)
     sc, si = codes.sort()
-    R = lsh_m.LSH()
-    R.alloc(K, L, 1, Hq, Hkv, bsz, M)
-    for b in range(bsz):
-        R.fill(0, b, sc[b].contiguous(), si[b].int().contiguous())
-    query = torch.randint(0, NB, (bsz * Hq, L), generator=g, dtype=torch.int32)
-    results = torch.zeros((bsz * Hq, M), dtype=torch.int32)
-    nnz = torch.zeros((bsz * Hq,), dtype=torch.int32)
-    R.batch_retrieve(0, query, results, nnz)
-    mask = R.get_mask().clone().view(torch.uint8).reshape(bsz * Hq, M)
     for b in range(bsz):
         T = oracle.Tables(Hkv, L, K, M)
         T.fill(sc[b].contiguous(), si[b].int().contiguous())
@@ -228,26 +226,14 @@ def test_port_probe_vs_live_reference(K, L, seq, delta, group, bsz):
         assert torch.equal((cnt > 1).sum(-1).int(), nz)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="oracle/_ref not built / CPU lacks AVX-512")
 def test_port_attention_vs_live_reference():
-    _, sa_m, _ = ref_loader.load()
-    g = torch.Generator().manual_seed(77)
-    B, Hq, Hkv, d, K, L, n, M = 1, 8, 2, 128, 10, 150, 2048, 2048 + 128
-    key = torch.randn((B, Hkv, n, d), generator=g).bfloat16()
-    value = torch.randn((B, Hkv, n, d), generator=g).bfloat16()
-    kn = key.norm(p=2, dim=-1).float()
-    q = torch.randn((B * Hq, d), generator=g).bfloat16()
-    nnz = torch.randint(1, n, (B * Hq,), generator=g).int()
-    ind = torch.zeros((B * Hq, M), dtype=torch.int32)
-    for h in range(B * Hq):
-        ind[h, : nnz[h]] = torch.randperm(n, generator=g)[: nnz[h]].int()
-    S = sa_m.SparseAttentionServer()
-    S.alloc(1, Hq, Hkv, d, B, M)
-    S.fill(0, 0, key[0].contiguous(), value[0].contiguous(), kn[0].contiguous())
-    out_ref = torch.zeros((B * Hq, d), dtype=torch.bfloat16)
-    mve_ref = torch.zeros((2, B * Hq))
+    """SparseAttentionServer.attention_wrapper's recorded outputs (tests/golden/operator_cases.npz) vs the port."""
+    B, Hq, Hkv, d, K, L, n, M = (ATTN_DIMS[k] for k in ("B", "Hq", "Hkv", "d", "K", "L", "n", "M"))
+    key, value, kn, q, nnz, ind = attention_case_inputs()
+    ref = load_operator_case("attn", key, value, kn, q, nnz, ind)
+    out_ref = bf16_from_u16(ref["out_bf16"]).reshape(B * Hq, d)
+    mve_ref = torch.from_numpy(ref["mve"])
     qn = q.float().norm(p=2, dim=-1)
-    S.attention_wrapper(0, K, L, out_ref, mve_ref, q, qn, ind, nnz)
     t = dict(B=B, Hkv=Hkv, n=n, d=d, M=M, key=key, value=value, key_norm=kn)
     k, v, knp = pad_store(t)
     out, mve, _ = oracle.attention_wrapper(k, v, knp, K, L, q, qn, ind, nnz)

@@ -1,5 +1,6 @@
-"""Drop-in proof, CPU container only: the reference's own sources are parsed (never imported -- they need FlashInfer and
-the compiled pybind modules) and every name, keyword and positional order they use must bind against this repo's mirrors.
+"""Drop-in proof: every name, keyword and positional order the reference's sources use must bind against this repo's
+mirrors.  The reference's call surface was read from its sources (never imported -- they need FlashInfer and the compiled
+pybind modules) into tests/golden/reference_api.json by tests/golden/make_golden.py.
 
   * `models/attnserver.py` class LSHSparseAttnServer (reference :7-331): constructor parameters with defaults and the
     seven methods with their parameter names -> `magicpig_b200.attnserver.LSHSparseAttnServer`.
@@ -10,18 +11,15 @@ the compiled pybind modules) and every name, keyword and positional order they u
     `SparseAttentionServer`: same method names, same parameter order.
   * `models/attnserver.py` itself drives the two operator classes (`:51-53, 172, 193, 299-300, 329-330`): those calls
     must bind against the mirrors too.
-
-Skips cleanly where /root/reference is absent (the GPU box).
 """
-import ast
 import inspect
+import json
 import os
-import re
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this host")
+with open(os.path.join(os.path.dirname(__file__), "golden", "reference_api.json")) as _f:
+    API = json.load(_f)
 
 # reference entry points deliberately not mirrored, with the SURVEY.md row that scopes them out
 EXCLUDED = {
@@ -30,27 +28,11 @@ EXCLUDED = {
 }
 
 
-def _parse(path):
-    with open(os.path.join(REF, path)) as f:
-        return ast.parse(f.read())
-
-
-def _class(tree, name):
-    for node in ast.walk(tree):
-        if isinstance(node, ast.ClassDef) and node.name == name:
-            return node
-    raise AssertionError(f"class {name} not found")
-
-
-def _methods(cls):
-    return {n.name: n for n in cls.body if isinstance(n, ast.FunctionDef)}
-
-
-def _bind_call(sig: inspect.Signature, call: ast.Call, bound_method: bool):
+def _bind_call(sig: inspect.Signature, call: dict, bound_method: bool):
     """Replay a reference call (positional count + keyword names) on a mirror signature."""
-    args = [object()] * len(call.args)
-    kwargs = {k.arg: object() for k in call.keywords}
-    assert None not in kwargs, "reference call uses **kwargs"
+    args = [object()] * call["n_args"]
+    assert None not in call["keywords"], "reference call uses **kwargs"
+    kwargs = {k: object() for k in call["keywords"]}
     if not bound_method:
         args = [object()] + args  # self
     sig.bind(*args, **kwargs)  # raises TypeError on any mismatch
@@ -59,25 +41,22 @@ def _bind_call(sig: inspect.Signature, call: ast.Call, bound_method: bool):
 def test_attnserver_class_signature():
     from magicpig_b200.attnserver import LSHSparseAttnServer as Ours
 
-    ref = _methods(_class(_parse("models/attnserver.py"), "LSHSparseAttnServer"))
+    ref = API["attnserver_methods"]
     assert set(ref) == {"__init__", "alloc_buffer", "fill", "build_table", "plan", "decode", "clear"}
     for name, fn in ref.items():
         assert hasattr(Ours, name), f"mirror lacks method {name}"
         ours = list(inspect.signature(getattr(Ours, name)).parameters.values())
-        theirs = [a.arg for a in fn.args.args]
+        theirs = fn["args"]
         # same names in the same positions (the mirror may append extra keywords after the reference's)
         assert [p.name for p in ours[: len(theirs)]] == theirs, (name, theirs, [p.name for p in ours])
         # defaults of the reference constructor carry over literally
-        defaults = fn.args.defaults
-        for a, dflt in zip(fn.args.args[len(fn.args.args) - len(defaults):], defaults):
-            p = next(p for p in ours if p.name == a.arg)
-            assert p.default is not inspect.Parameter.empty, f"{name}({a.arg}) lost its default"
-            try:
-                want = ast.literal_eval(dflt)
-            except ValueError:
+        for dflt in fn["defaults"]:
+            p = next(p for p in ours if p.name == dflt["arg"])
+            assert p.default is not inspect.Parameter.empty, f"{name}({dflt['arg']}) lost its default"
+            if not dflt["literal"]:
                 continue  # torch.bfloat16
             got = list(p.default) if isinstance(p.default, tuple) else p.default
-            assert got == want, (name, a.arg, got, want)
+            assert got == dflt["value"], (name, dflt["arg"], got, dflt["value"])
         # anything the mirror adds must be optional
         for p in ours[len(theirs):]:
             assert p.default is not inspect.Parameter.empty, f"{name}: extra parameter {p.name} has no default"
@@ -86,38 +65,13 @@ def test_attnserver_class_signature():
 def test_llama_call_sites_bind():
     from magicpig_b200.attnserver import LSHSparseAttnServer as Ours
 
-    tree = _parse("models/llama.py")
     seen = set()
-    for node in ast.walk(tree):
-        if not isinstance(node, ast.Call):
-            continue
-        f = node.func
-        if isinstance(f, ast.Name) and f.id == "LSHSparseAttnServer":                     # llama.py:92-93
-            _bind_call(inspect.signature(Ours.__init__), node, bound_method=False)
-            seen.add("__init__")
-        elif (isinstance(f, ast.Attribute) and isinstance(f.value, ast.Attribute) and f.value.attr == "attention_server"):
-            assert hasattr(Ours, f.attr), f"llama.py calls attention_server.{f.attr}"
-            _bind_call(inspect.signature(getattr(Ours, f.attr)), node, bound_method=False)
-            seen.add(f.attr)
+    for call in API["llama_calls"]:   # llama.py:92-93 constructor, attention_server.<method>(...) elsewhere
+        name = call["method"]
+        assert hasattr(Ours, name), f"llama.py calls attention_server.{name}"
+        _bind_call(inspect.signature(getattr(Ours, name)), call, bound_method=False)
+        seen.add(name)
     assert seen == {"__init__", "decode", "build_table", "fill", "plan", "alloc_buffer", "clear"}, seen
-
-
-def _pybind_defs(path):
-    with open(os.path.join(REF, path)) as f:
-        return re.findall(r'\.def\("([a-z_0-9]+)"', f.read())
-
-
-def _cpp_members(path, cls):
-    """method name -> parameter names (without the `_pt` suffix the reference gives tensor arguments)."""
-    with open(os.path.join(REF, path)) as f:
-        text = f.read()
-    body = text[text.index(f"class {cls}"):]
-    body = body[: body.index("private:")]
-    out = {}
-    for m in re.finditer(r"(?:void|torch::Tensor|int)\s+([a-z_0-9]+)\(([^)]*)\);", body):
-        params = [p.strip().split()[-1] for p in m.group(2).split(",") if p.strip()]
-        out[m.group(1)] = [re.sub(r"_pt$", "", p) for p in params]
-    return out
 
 
 @pytest.mark.parametrize("cc,hdr,cls", [
@@ -128,8 +82,8 @@ def test_operator_mirrors_cover_pybind_surface(cc, hdr, cls):
     from magicpig_b200 import ops
 
     Ours = getattr(ops, cls)
-    defs = _pybind_defs(cc)
-    members = _cpp_members(hdr, cls)
+    defs = API["pybind_defs"][cc]
+    members = API["cpp_members"][hdr][cls]
     assert len(defs) >= 7
     for name in defs:
         if name in EXCLUDED:
@@ -147,13 +101,10 @@ def test_attnserver_operator_calls_bind():
     from magicpig_b200 import ops
 
     owner = {"attn_server": ops.SparseAttentionServer, "lsh_retriever": ops.LSH}
-    tree = _class(_parse("models/attnserver.py"), "LSHSparseAttnServer")
     n = 0
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute) and isinstance(node.func.value, ast.Attribute) \
-                and node.func.value.attr in owner:
-            Ours = owner[node.func.value.attr]
-            assert hasattr(Ours, node.func.attr), (node.func.value.attr, node.func.attr)
-            _bind_call(inspect.signature(getattr(Ours, node.func.attr)), node, bound_method=False)
-            n += 1
+    for call in API["attnserver_operator_calls"]:
+        Ours = owner[call["owner"]]
+        assert hasattr(Ours, call["method"]), (call["owner"], call["method"])
+        _bind_call(inspect.signature(getattr(Ours, call["method"])), call, bound_method=False)
+        n += 1
     assert n >= 7, n
